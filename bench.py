@@ -1,6 +1,7 @@
 """Headline benchmark: Flux denoise it/s (BASELINE.json metric) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c4|c5] [--impl ours|reference|reference-gpu]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 A "step" is one denoise step of the hot path (Flux.forward over all 19+38 blocks + the Euler update) for one sample
@@ -15,6 +16,12 @@ per GPU (batch-parallel across GPUs, weak scaling).  Default workload = BASELINE
 Weights are synthetic (seeded N(0, 0.02^2), quantised with the reference flow, input scales calibrated by >= 13 eager
 steps on rank 0 and replicated with one NCCL broadcast); latents / text embeddings are synthetic tensors of the
 published shapes.
+
+--dump-outputs DIR writes the latent the timed loop returned after its last step (what a caller of
+DenoiseSession.step_device receives) to DIR/latent.npy (DIR/latent_rank<r>.npy with several GPUs), float32.  Weights
+and inputs are seeded, so two builds run with the same arguments can be compared output for output.  It covers
+--impl ours only and is refused with the other arms: those time the reference's own modules as a baseline (a bounded
+block sample on the host CPU, or a child process on the GPU), which do not change with this package's builds.
 
 One JSON line on stdout (rank 0):
   value         sample-steps/s over all GPUs, latents resident in HBM (CUDA-graph replay per step)
@@ -640,7 +647,13 @@ def main():
     ap.add_argument("--no-vae", action="store_true",
                     help="skip the VAE decode and text-encoder measurements (SURVEY 8f N4) beside the metric")
     ap.add_argument("--no-graph", action="store_true", help="launch kernels eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the latent of the last timed step as DIR/latent.npy (float32; --impl ours only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     cfg = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -719,11 +732,11 @@ def main():
         PAR.barrier()
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
-        step_fn(steps)
+        out = step_fn(steps)
         e.record()
         torch.cuda.synchronize()
         PAR.barrier()
-        return PAR.max_over_ranks(s.elapsed_time(e), dev)
+        return PAR.max_over_ranks(s.elapsed_time(e), dev), out
 
     # ---- value: latents resident in HBM
     def device_steps(k):
@@ -734,8 +747,15 @@ def main():
 
     device_steps(args.warmup)
     with ClockSampler(local_rank) as clocks:
-        ms_total = timed_loop(device_steps, args.steps)
+        ms_total, latent = timed_loop(device_steps, args.steps)
     clock_info = clocks.summary()
+    if args.dump_outputs:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = "latent.npy" if world == 1 else f"latent_rank{rank}.npy"
+        np.save(os.path.join(args.dump_outputs, name), latent.float().cpu().numpy())
+    del latent
     ms_per_step = ms_total / args.steps
     value = world * 1000.0 / ms_per_step
 
@@ -750,7 +770,7 @@ def main():
         return h
 
     host_steps(2)
-    e2e_ms = timed_loop(host_steps, args.steps) / args.steps
+    e2e_ms = timed_loop(host_steps, args.steps)[0] / args.steps
     e2e_value = world * 1000.0 / e2e_ms
 
     # ---- roofline: CUDA events around every kernel launch of an eager-launch pass + the measured FP8 ceiling

@@ -404,13 +404,13 @@ def test_layernorm_fused_into_the_gemm_launch_is_bit_identical(lib, res, batch):
 
 def test_prequantised_safetensors_roundtrip_and_the_reference_loads_it(gold, golden_dir, tmp_path, cpu_semantics):
     """pipeline.save_prequantized writes ONE safetensors file in the reference's key layout: load_prequantized brings
-    back a frozen, graph-capturable model with bit-identical outputs, and -- when the staged reference is present -- the
-    reference's own Flux(prequantized_flow=True) loads the same file the way util.load_flow_model does
-    (load_sft + load_state_dict(assign=True), util.py:245-256) and runs it on its library kernels."""
+    back a frozen, graph-capturable model with bit-identical outputs; the file holds exactly the keys, dtypes and shapes
+    of the reference-minted state, so the reference's own Flux(prequantized_flow=True) loads it the way
+    util.load_flow_model does (load_sft + load_state_dict(assign=True), util.py:245-256), and what the reference computes
+    from this file on its library kernels (stored by oracle/reference_golden.py) matches ours."""
     from safetensors.torch import load_file
 
     from flux_fp8_api_b200 import model as M, pipeline as PL
-    from oracle import ref_loader as R
 
     net = tiny_net(gold)
     inp = {k: v.to(DEV) for k, v in gold["inputs"].items()}
@@ -427,17 +427,9 @@ def test_prequantised_safetensors_roundtrip_and_the_reference_loads_it(gold, gol
         req = {k: v for k, v in inp.items() if k != "timesteps"}
         assert torch.equal(PL.DenoiseSession(back, req).step_device(req["img"], sched[0], sched[1]),
                            PL.DenoiseSession(net, req).step_device(req["img"], sched[0], sched[1]))
-    if not R.available():
-        pytest.skip("oracle/_ref not staged: the reference-side load is checked where it is")
-    ref = R.load()
-    with torch.device("meta"):
-        theirs = ref.fm.Flux(R.model_spec(ref, gold["tiny"], prequantized_flow=True), dtype=BF16)
     sd = load_file(path, device="cpu")
-    missing, unexpected = theirs.load_state_dict(sd, strict=False, assign=True)
-    assert not missing and not unexpected
-    theirs = theirs.to(DEV).eval()
-    assert R.all_frozen(ref, theirs)
-    with torch.inference_mode():
-        y_ref = theirs(**inp)
+    assert {k: (v.dtype, v.shape) for k, v in sd.items()} == {k: (v.dtype, v.shape) for k, v in gold["state"].items()}
+    assert all(torch.equal(sd[k], v) for k, v in gold["state"].items())
+    y_ref = torch.load(os.path.join(golden_dir, "reference_tiny_gpu.pt"))["y_ref"]
     assert maxdiff(y_ref, y) <= 2.0 ** -4
     assert maxdiff(y_ref, gold["y_fp8"]) <= 2.0 ** -4

@@ -1,6 +1,6 @@
 """GPU (-m gpu): the VAE decode kernels (SURVEY.md 8f N4) against torch fp32 references of the same ops, the oracle's
-golden vectors, and the UNMODIFIED reference AutoEncoder (staged under oracle/_ref) run on the same B200 under
-torch.autocast("cuda", torch.bfloat16) exactly as flux_pipeline.py:423-438 runs it."""
+golden vectors, and the outputs of the UNMODIFIED reference AutoEncoder run on a B200 under torch.autocast("cuda",
+torch.bfloat16) exactly as flux_pipeline.py:423-438 runs it, and in fp32 (stored by oracle/reference_golden.py)."""
 import json
 import math
 import os
@@ -11,13 +11,12 @@ import torch.nn.functional as F
 
 from flux_fp8_api_b200 import autoencoder as A
 from flux_fp8_api_b200 import ops
-from oracle import ref_loader as R
+from oracle import reference_golden as G
 from oracle import vae_oracle as V
 
 pytestmark = pytest.mark.gpu
 BF16 = torch.bfloat16
 DEV = "cuda"
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ULP = 2.0 ** -7  # one bf16 ulp relative to a value's binade top
 
 
@@ -200,58 +199,58 @@ def test_loud_failures():
         ops.conv2d_nhwc(x.new_zeros((1, 8, 8, 64)), _rand((64, 64), 44), None, 1, stride=2)  # stride 2 is the 3x3 Downsample only
 
 
-@pytest.mark.skipif(not R.available(), reason="oracle/_ref not staged (python oracle/fetch_ref.py)")
+def _ours(state_seed, prefixes=("decoder.",)):
+    """Flux's VAE (ch 128, ch_mult 1-2-4-4) with the seeded state oracle/reference_golden.py gave the reference, and the
+    byte checksum of that state."""
+    ours = A.AutoEncoder(A.AutoEncoderParams(**G.VAE_PARAMS))
+    sd = V.synthetic_state(ours, seed=state_seed, prefixes=prefixes)
+    ours.load_state_dict(sd, strict=prefixes != ("decoder.",))
+    return ours.to(DEV, BF16).eval(), G.state_bytesum(sd)
+
+
+def _timed(fn, n=3):
+    fn()
+    torch.cuda.synchronize()
+    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    s.record()
+    for _ in range(n):
+        out = fn()
+    e.record()
+    torch.cuda.synchronize()
+    return out, s.elapsed_time(e) / n
+
+
+def _against_the_stored_reference(golden_dir, case, state_sum, inputs, out, ours_key, ref_key, ref32_key):
+    """|ours - reference fp32| and |ours - reference bf16 autocast| against the reference's own bf16-vs-fp32 distance,
+    all on the sample of positions the reference's outputs were stored at (G.sample: spread over every row, column and
+    channel).  The state and input checksums come first, so a change to how they are generated names itself."""
+    gold = torch.load(os.path.join(golden_dir, "reference_vae_full.pt"))[case]
+    assert state_sum == gold["state_bytesum"], f"{case}: the seeded VAE state differs from the one the reference ran"
+    assert G.state_bytesum(inputs) == gold["inputs_bytesum"], f"{case}: the input differs from the one the reference ran"
+    assert list(out.shape) == gold["shape"] and out.dtype == BF16
+    ref, ref32 = gold[ref_key].float(), gold[ref32_key].float()
+    mine = G.sample(out, ref.numel()).float()
+    floor, d32, d_ref = (ref - ref32).abs(), (mine - ref32).abs(), (mine - ref).abs()
+    rep = {"case": case, "reference_autocast_vs_fp32": {"mean": floor.mean().item(), "max": floor.max().item(),
+                                                        "mean_whole": gold["floor_mean"], "max_whole": gold["floor_max"]},
+           f"{ours_key}_vs_fp32": {"mean": d32.mean().item(), "max": d32.max().item()},
+           f"{ours_key}_vs_reference_autocast": {"mean": d_ref.mean().item(), "max": d_ref.max().item()}}
+    return floor, d32, d_ref, rep
+
+
 @pytest.mark.parametrize("res", [1024, 768, 1536])
-def test_full_size_decode_against_the_reference_on_this_gpu(res):
-    """Flux's VAE (ch 128, ch_mult 1-2-4-4) at full resolution: ours vs the staged reference under CUDA autocast, with the
-    reference's own bf16-vs-fp32 distance as the floor; both timed with CUDA events."""
-    ref = R.load()
-    if ref.ae is None:
-        pytest.skip("modules/autoencoder.py not staged (re-run oracle/fetch_ref.py)")
-    params = dict(resolution=256, in_channels=3, ch=128, out_ch=3, ch_mult=[1, 2, 4, 4], num_res_blocks=2, z_channels=16,
-                  scale_factor=0.3611, shift_factor=0.1159)
-    rae = ref.ae.AutoEncoder(ref.ae.AutoEncoderParams(**params))
-    sd = V.synthetic_state(rae, seed=77)
-    rae.load_state_dict(sd, strict=False)
-    rae = rae.to(DEV, BF16).eval()  # util.py:287: the reference keeps the VAE in bf16
-    ours = A.AutoEncoder(A.AutoEncoderParams(**params))
-    ours.load_state_dict(sd, strict=False)
-    ours = ours.to(DEV, BF16).eval()
-    z = torch.randn(1, 16, res // 8, res // 8, device=DEV, generator=torch.Generator(device=DEV).manual_seed(78)) * 1.2
-
-    def timed(fn, n=3):
-        fn()
-        torch.cuda.synchronize()
-        s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        s.record()
-        for _ in range(n):
-            out = fn()
-        e.record()
-        torch.cuda.synchronize()
-        return out, s.elapsed_time(e) / n
-
+def test_full_size_decode_against_the_reference_on_this_gpu(res, golden_dir):
+    """Flux's VAE (ch 128, ch_mult 1-2-4-4) at full resolution: ours vs the reference's decode under CUDA autocast and in
+    fp32, as oracle/reference_golden.py stored them from the unmodified reference on a B200, with the reference's own
+    bf16-vs-fp32 distance as the floor; ours timed with CUDA events."""
+    ours, state_sum = _ours(77)
+    z = G.vae_decode_latent(78, 1, res, res)
     with torch.inference_mode():
-        def run_ref():
-            with torch.autocast(device_type="cuda", dtype=BF16, cache_enabled=False):  # flux_pipeline.py:431-434
-                return rae.decode(z)
-
-        y_ref, ms_ref = timed(run_ref)
-        y_ours, ms_ours = timed(lambda: ours.decode(z))
-        rae32 = rae.float()
-        y32 = rae32.decode(z)
-    assert y_ours.shape == y_ref.shape == (1, 3, res, res) and y_ours.dtype == BF16
-    floor = (y_ref.float() - y32).abs()
-    d_ref = (y_ours.float() - y_ref.float()).abs()
-    d_32 = (y_ours.float() - y32).abs()
-    rep = {"res": res, "amax": y32.abs().max().item(), "rms": y32.pow(2).mean().sqrt().item(),
-           "reference_autocast_vs_fp32": {"mean": floor.mean().item(), "max": floor.max().item()},
-           "ours_vs_fp32": {"mean": d_32.mean().item(), "max": d_32.max().item()},
-           "ours_vs_reference_autocast": {"mean": d_ref.mean().item(), "max": d_ref.max().item()},
-           "ms_reference_autocast": ms_ref, "ms_ours": ms_ours}
+        y_ours, ms_ours = _timed(lambda: ours.decode(z))
+    floor, d_32, d_ref, rep = _against_the_stored_reference(golden_dir, f"decode-{res}", state_sum, {"z": z}, y_ours, "ours",
+                                                            "y_ref", "y32")
+    rep["ms_ours"] = ms_ours
     print(json.dumps(rep))
-    os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-    with open(os.path.join(ROOT, "gpurun_out", f"vae_parity_{res}.json"), "w") as f:
-        json.dump(rep, f, indent=1)
     assert torch.isfinite(y_ours).all()
     # as close to the fp32 answer as the reference's own bf16 run is (25 % slack: two bf16 runs are not the same run)
     assert d_32.mean().item() <= 1.25 * floor.mean().item()
@@ -260,35 +259,19 @@ def test_full_size_decode_against_the_reference_on_this_gpu(res):
     assert d_ref.mean().item() <= 1.5 * floor.mean().item()
 
 
-@pytest.mark.skipif(not R.available(), reason="oracle/_ref not staged (python oracle/fetch_ref.py)")
 @pytest.mark.parametrize("B,height,width", [(5, 128, 192), (2, 720, 1280)])
-def test_decoder_shapes_outside_the_fast_paths_against_the_reference(B, height, width):
+def test_decoder_shapes_outside_the_fast_paths_against_the_reference(B, height, width, golden_dir):
     """Batch 5 (more images than the convolution epilogue keeps statistics for: the GroupNorms reduce by themselves) and a
     720 x 1280 image (latent 90 x 160: strips of 32 pixels, rows clipped, 14 400 attention positions) -- same bars as the
-    full-size test, against the staged reference under CUDA autocast."""
-    ref = R.load()
-    if ref.ae is None:
-        pytest.skip("modules/autoencoder.py not staged (re-run oracle/fetch_ref.py)")
-    params = dict(resolution=256, in_channels=3, ch=128, out_ch=3, ch_mult=[1, 2, 4, 4], num_res_blocks=2, z_channels=16,
-                  scale_factor=0.3611, shift_factor=0.1159)
-    rae = ref.ae.AutoEncoder(ref.ae.AutoEncoderParams(**params))
-    sd = V.synthetic_state(rae, seed=91)
-    rae.load_state_dict(sd, strict=False)
-    rae = rae.to(DEV, BF16).eval()
-    ours = A.AutoEncoder(A.AutoEncoderParams(**params))
-    ours.load_state_dict(sd, strict=False)
-    ours = ours.to(DEV, BF16).eval()
-    z = torch.randn(B, 16, height // 8, width // 8, device=DEV, generator=torch.Generator(device=DEV).manual_seed(92)) * 1.2
+    full-size test, against the stored reference outputs."""
+    ours, state_sum = _ours(91)
+    z = G.vae_decode_latent(92, B, height, width)
     with torch.inference_mode():
-        with torch.autocast(device_type="cuda", dtype=BF16, cache_enabled=False):
-            y_ref = rae.decode(z)
         y = ours.decode(z)
-        y32 = rae.float().decode(z)
     assert y.shape == (B, 3, height, width)
-    floor = (y_ref.float() - y32).abs()
-    d32 = (y.float() - y32).abs()
-    print(f"{B} x {height}x{width}: reference bf16-vs-fp32 mean {floor.mean().item():.4g} max {floor.max().item():.4g}; "
-          f"ours-vs-fp32 mean {d32.mean().item():.4g} max {d32.max().item():.4g}")
+    floor, d32, _, rep = _against_the_stored_reference(golden_dir, f"decode-{B}x{height}x{width}", state_sum, {"z": z}, y,
+                                                       "ours", "y_ref", "y32")
+    print(json.dumps(rep))
     assert torch.isfinite(y).all()
     assert d32.mean().item() <= 1.25 * floor.mean().item() and d32.max().item() <= 1.5 * floor.max().item()
 
@@ -359,55 +342,21 @@ def test_tiny_encoder_against_the_golden_moments(golden_dir):
     assert z.shape == (2, 16, 8, 8) and torch.isfinite(z).all()
 
 
-@pytest.mark.skipif(not R.available(), reason="oracle/_ref not staged (python oracle/fetch_ref.py)")
-def test_full_size_encode_against_the_reference_on_this_gpu():
-    """Flux's VAE encoder at 1024 x 1024 (img2img, flux_pipeline.py:489-500): the Gaussian's moments against the staged reference
-    under CUDA autocast with its own bf16-vs-fp32 distance as the floor; the sampled latent with the same torch seed."""
-    ref = R.load()
-    if ref.ae is None:
-        pytest.skip("modules/autoencoder.py not staged (re-run oracle/fetch_ref.py)")
-    params = dict(resolution=256, in_channels=3, ch=128, out_ch=3, ch_mult=[1, 2, 4, 4], num_res_blocks=2, z_channels=16,
-                  scale_factor=0.3611, shift_factor=0.1159)
-    rae = ref.ae.AutoEncoder(ref.ae.AutoEncoderParams(**params))
-    sd = V.synthetic_state(rae, seed=93, prefixes=("decoder.", "encoder."))
-    rae.load_state_dict(sd, strict=True)
-    rae = rae.to(DEV, BF16).eval()
-    ours = A.AutoEncoder(A.AutoEncoderParams(**params))
-    ours.load_state_dict(sd, strict=True)
-    ours = ours.to(DEV, BF16).eval()
-    img = (torch.rand(1, 3, 1024, 1024, device=DEV, generator=torch.Generator(device=DEV).manual_seed(94)) * 2 - 1).to(BF16)
-
-    def timed(fn, n=3):
-        fn()
-        torch.cuda.synchronize()
-        s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        s.record()
-        for _ in range(n):
-            out = fn()
-        e.record()
-        torch.cuda.synchronize()
-        return out, s.elapsed_time(e) / n
-
+def test_full_size_encode_against_the_reference_on_this_gpu(golden_dir):
+    """Flux's VAE encoder at 1024 x 1024 (img2img, flux_pipeline.py:489-500): the Gaussian's moments against the reference's
+    under CUDA autocast and in fp32 (stored by oracle/reference_golden.py), with its own bf16-vs-fp32 distance as the
+    floor; the sampled latent's shape."""
+    ours, state_sum = _ours(G.VAE_ENCODE_SEEDS[0], prefixes=("decoder.", "encoder."))
+    img = G.vae_encode_image(G.VAE_ENCODE_SEEDS[1])
     with torch.inference_mode():
-        def run_ref():
-            with torch.autocast(device_type="cuda", dtype=BF16, cache_enabled=False):
-                return rae.encoder(img)
-
-        m_ref, ms_ref = timed(run_ref)
-        m_ours, ms_ours = timed(lambda: ours.encoder(img))
+        m_ours, ms_ours = _timed(lambda: ours.encoder(img))
         torch.manual_seed(11)
         with torch.autocast(device_type="cuda", dtype=BF16, cache_enabled=False):
-            z_ref = rae.encode(img)
-            torch.manual_seed(11)
             z_ours = ours.encode(img)
-        m32 = rae.float().encoder(img.float())
-    floor, d32 = (m_ref.float() - m32).abs(), (m_ours.float() - m32).abs()
-    rep = {"moments_amax": m32.abs().max().item(), "reference_autocast_vs_fp32": {"mean": floor.mean().item(), "max": floor.max().item()},
-           "ours_vs_fp32": {"mean": d32.mean().item(), "max": d32.max().item()},
-           "latent_ours_vs_reference": {"mean": (z_ours.float() - z_ref.float()).abs().mean().item()},
-           "ms_reference_autocast": ms_ref, "ms_ours": ms_ours}
+    assert m_ours.shape == (1, 32, 128, 128) and z_ours.shape == (1, 16, 128, 128)
+    floor, d32, _, rep = _against_the_stored_reference(golden_dir, "encode-1024", state_sum, {"img": img}, m_ours, "moments",
+                                                       "m_ref", "m32")
+    rep["ms_ours"] = ms_ours
     print(json.dumps(rep))
-    with open(os.path.join(ROOT, "gpurun_out", "vae_encode_parity_1024.json"), "w") as f:
-        json.dump(rep, f, indent=1)
-    assert m_ours.shape == m_ref.shape == (1, 32, 128, 128) and z_ours.shape == (1, 16, 128, 128)
+    assert torch.isfinite(z_ours).all()
     assert d32.mean().item() <= 1.25 * floor.mean().item() and d32.max().item() <= 1.5 * floor.max().item()

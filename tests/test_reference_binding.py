@@ -1,7 +1,8 @@
 """The reference-side binding (flux_fp8_api_b200.reference_binding, quoted in INTEGRATION.md) executed against the
-staged UNMODIFIED reference (oracle/_ref, see oracle/fetch_ref.py).
+staged UNMODIFIED reference (oracle/_ref, see oracle/fetch_ref.py); the signature and state-layout checks run against the
+reference's surface stored in tests/golden/reference_surface.json.
 
-CPU part: the staged files are byte-identical to /root/reference; after bind() the reference's own `Flux` container
+CPU part: the staged files are byte-identical to the reference tree they were staged from; after bind() the reference's own `Flux` container
 builds over the B200 classes, has exactly the reference's state-dict keys, and loads a reference-minted prequantised
 state dict.  GPU part (-m gpu): that container -- the reference's own Flux.forward driving our blocks -- gives the same
 output as this package's Flux and matches the reference-minted golden; LoRA load / unload through the reference-named
@@ -43,27 +44,25 @@ def test_staged_reference_is_the_unmodified_reference():
     assert tracked == ""
 
 
-@needs_ref
-def test_autoencoder_surface_matches_the_reference():
-    """Constructor signatures, state-dict keys and shapes of the decode half (SURVEY.md 8f N4)."""
+def test_autoencoder_surface_matches_the_reference(golden_dir):
+    """Constructor signatures, state-dict keys and shapes of the decode half (SURVEY.md 8f N4), against the reference's
+    as stored in tests/golden/reference_surface.json (oracle/reference_golden.py)."""
     import inspect
+    import json
 
     from flux_fp8_api_b200 import autoencoder as A
 
-    ref = R.load()
-    assert ref.ae is not None, getattr(ref, "ae_error", "")
-    for name in ("AttnBlock", "ResnetBlock", "Upsample", "Downsample", "Encoder", "Decoder", "DiagonalGaussian", "AutoEncoder"):
-        ours, theirs = getattr(A, name), getattr(ref.ae, name)
-        assert [p.name for p in inspect.signature(ours.__init__).parameters.values()] == \
-               [p.name for p in inspect.signature(theirs.__init__).parameters.values()], name
-    assert set(A.AutoEncoderParams.model_fields) == set(ref.ae.AutoEncoderParams.model_fields)
-    params = dict(resolution=64, in_channels=3, ch=64, out_ch=3, ch_mult=[1, 2, 4, 4], num_res_blocks=2, z_channels=16,
-                  scale_factor=0.3611, shift_factor=0.1159)
-    theirs = ref.ae.AutoEncoder(ref.ae.AutoEncoderParams(**params)).state_dict()
+    with open(os.path.join(golden_dir, "reference_surface.json")) as f:
+        gold = json.load(f)
+    for name, theirs in gold["autoencoder_init"].items():
+        assert [p.name for p in inspect.signature(getattr(A, name).__init__).parameters.values()] == theirs, name
+    assert sorted(A.AutoEncoderParams.model_fields) == gold["autoencoder_params_fields"]
+    params, theirs = gold["autoencoder_state_shapes"]["params"], gold["autoencoder_state_shapes"]["shapes"]
     ours = A.AutoEncoder(A.AutoEncoderParams(**params)).state_dict()
-    assert {k: v.shape for k, v in ours.items()} == {k: v.shape for k, v in theirs.items()}
-    # a reference checkpoint loads the way util.py:285 loads it
-    missing, unexpected = A.AutoEncoder(A.AutoEncoderParams(**params)).load_state_dict(theirs, strict=False)
+    assert {k: list(v.shape) for k, v in ours.items()} == theirs
+    # a reference checkpoint (its keys and shapes) loads the way util.py:285 loads it
+    ckpt = {k: torch.zeros(shape) for k, shape in theirs.items()}
+    missing, unexpected = A.AutoEncoder(A.AutoEncoderParams(**params)).load_state_dict(ckpt, strict=False)
     assert not missing and not unexpected
 
 
@@ -93,25 +92,28 @@ def test_bind_redirects_the_autoencoder_and_a_reference_checkpoint_loads():
     assert ref.ae.AutoEncoder is orig
 
 
-@needs_ref
-def test_signatures_match_the_reference():
+def test_signatures_match_the_reference(golden_dir):
+    """Every replaced reference function / class / Flux method keeps the reference's signature, as stored in
+    tests/golden/reference_surface.json (oracle/reference_golden.py)."""
     import inspect
+    import json
 
     from flux_fp8_api_b200 import blocks, f8linear, model
 
-    ref = R.load()
+    with open(os.path.join(golden_dir, "reference_surface.json")) as f:
+        theirs = json.load(f)["signatures"]
 
     def params(fn):
-        return [(p.name, p.kind, p.default if not isinstance(p.default, torch.dtype) else str(p.default))
+        return [[p.name, int(p.kind), repr(p.default) if not isinstance(p.default, torch.dtype) else str(p.default)]
                 for p in inspect.signature(fn).parameters.values()]
 
     for name in ("F8Linear", "recursive_swap_linears", "quantize_flow_transformer_and_dispatch_float8"):
-        assert params(getattr(f8linear, name)) == params(getattr(ref.f8, name)), name
+        assert params(getattr(f8linear, name)) == theirs[f"float8_quantize.{name}"], name
     for name in ("attention", "rope", "apply_rope", "EmbedND", "QKNorm", "Modulation", "DoubleStreamBlock",
                  "SingleStreamBlock"):
-        assert params(getattr(blocks, name)) == params(getattr(ref.fm, name)), name
+        assert params(getattr(blocks, name)) == theirs[f"flux_model.{name}"], name
     for meth in ("get_lora", "has_lora", "load_lora", "unload_lora", "from_pretrained", "forward"):
-        assert [p[0] for p in params(getattr(model.Flux, meth))] == [p[0] for p in params(getattr(ref.fm.Flux, meth))], meth
+        assert [p[0] for p in params(getattr(model.Flux, meth))] == [p[0] for p in theirs[f"flux_model.Flux.{meth}"]], meth
     # block forwards: the reference's positional / keyword names first (extras are optional keyword hand-downs)
     assert [p[0] for p in params(blocks.DoubleStreamBlock.forward)][:5] == ["self", "img", "txt", "vec", "pe"]
     assert [p[0] for p in params(blocks.SingleStreamBlock.forward)][:4] == ["self", "x", "vec", "pe"]
